@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- TF-IDF + LSI(k=50) throughput on synthetic sparse ATAC (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--scaling weak|strong]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--scaling weak|strong] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 A "step" is one pass of the hot path -- mu.atac.pp.tfidf + mu.atac.tl.lsi -- over the whole synthetic matrix.
@@ -20,6 +20,10 @@ Prints ONE JSON line (rank 0):
   cfg3         (N = 8, or --cfg3 1) BASELINE configs[3]: LSI k=100 on 4M x 500k over 8 GPUs
 ``--impl reference`` times the CPU oracle (scipy restatement of the reference, oracle/) on the host cores; it never
 loads the CUDA library.
+
+``--dump-outputs DIR`` writes, after the timed steps, what the last main-leg step returned (TF-IDF values, LSI
+embedding, loadings and standard deviations) as DIR/<slot>.npy.  The synthetic matrix depends only on the arguments,
+so two builds run with the same arguments can be compared array for array (``dump_outputs``).
 """
 from __future__ import annotations
 
@@ -72,7 +76,15 @@ def parse():
     ap.add_argument("--mofa-iters", type=int, default=15)
     ap.add_argument("--mofa-k", type=int, default=30)
     ap.add_argument("--breakdown", action="store_true", help="one extra, synchronising step with phase timers")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned to its caller as DIR/<slot>.npy "
+                         "(fixed samples of the large arrays, under 64 MB in all; rank 0's cell shard when N > 1)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -235,15 +247,55 @@ def lsi_step_fn(ctx, A, k, tol):
     obs0 = pd.DataFrame(index=pd.RangeIndex(A.shape[0]).astype(str))
     var0 = pd.DataFrame(index=pd.RangeIndex(A.shape[1]).astype(str))
 
-    def step():
+    def step(keep=None):
+        """``keep``: a dict that receives the step's AnnData (the caller's view of the result) as keep["ad"]."""
+        if keep is not None:
+            keep.clear()                              # the previous step's result goes before this step allocates
         ad = mu.SimpleAnnData(A, obs=obs0, var=var0)  # counts stay untouched: tfidf writes a new matrix
         mu.atac.pp.tfidf(ad)
         info = mu.atac.tl.lsi(ad, n_comps=k, tol=tol, return_info=True)
         # leading singular values (stdev * sqrt(n-1), tools.py:65): the same global matrix must give the same
         # values on any number of GPUs (strong leg at N ranks vs main leg at 1 rank)
         info.sigma_head = [float(x) * float(np.sqrt(max(A.n_total - 1, 1))) for x in ad.uns["lsi"]["stdev"][:4]]
+        if keep is not None:
+            keep["ad"] = ad
         return info
     return step
+
+
+DUMP_BYTES = 16 << 20      # per dumped array: the four arrays of dump_outputs stay under 64 MB
+
+
+def dump_outputs(out_dir, ad):
+    """Write the slots one step of the main leg leaves for its caller, so that two builds can be compared output for
+    output.  Arrays up to DUMP_BYTES are written whole.  Of a larger one, a fixed sample of rows (seed 0, ascending
+    order) is written, so every run with the same arguments writes the same positions.
+      uns_lsi_stdev   uns["lsi"]["stdev"]                          (k,)
+      obsm_X_lsi      rows of obsm["X_lsi"]                         (cells, k)
+      varm_LSI        rows of varm["LSI"]                           (peaks, k)
+      X_data          stored TF-IDF values of X (kept in HBM)       (entries,)
+    The sign of each LSI component is arbitrary and can differ from run to run, so embedding and loading columns are
+    flipped together to make the largest-magnitude entry of each full loading column positive (the loadings are the
+    same on every rank).  Returns {name: shape}."""
+    import torch
+    rng = np.random.default_rng(0)
+
+    def rows(n, row_bytes):
+        m = max(1, DUMP_BYTES // row_bytes)
+        return np.arange(n) if n <= m else np.sort(rng.choice(n, m, replace=False))
+
+    X, emb, load = ad.X, ad.obsm["X_lsi"], ad.varm["LSI"]
+    sgn = np.where(load[np.abs(load).argmax(0), np.arange(load.shape[1])] < 0, -1, 1).astype(load.dtype)
+    pos = torch.from_numpy(rows(X.nnz, X.data.element_size())).to(X.device)
+    out = {"uns_lsi_stdev": ad.uns["lsi"]["stdev"],
+           "obsm_X_lsi": emb[rows(emb.shape[0], emb.itemsize * emb.shape[1])] * sgn,
+           "varm_LSI": load[rows(load.shape[0], load.itemsize * load.shape[1])] * sgn,
+           "X_data": X.data[pos].cpu().numpy()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+    return {name: list(a.shape) for name, a in out.items()}
 
 
 def spmm_roofline(ctx, kern, info, steps, nnz, n_local, D, k, clocks):
@@ -354,7 +406,13 @@ def main():
 
     # ---- main leg: device-resident counts -> tfidf -> lsi ------------------------------------------------------
     step = lsi_step_fn(ctx, A, k, args.tol)
-    ms_total, kern, launches, info, clocks = timed_steps(ctx, step, args.steps, args.warmup, sample_clocks=True)
+    last = {} if args.dump_outputs else None
+    ms_total, kern, launches, info, clocks = timed_steps(ctx, lambda: step(last), args.steps, args.warmup,
+                                                         sample_clocks=True)
+    if last is not None:
+        if rank == 0:
+            note("dump_outputs", {"dir": args.dump_outputs, "arrays": dump_outputs(args.dump_outputs, last["ad"])})
+        last.clear()
     value = n_total * args.steps / (ms_total / 1e3)
     roofline = spmm_roofline(ctx, kern, info, args.steps, nnz, n_local, D, k, clocks)
     pk, _ = peaks()

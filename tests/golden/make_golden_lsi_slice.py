@@ -7,9 +7,10 @@ the build container (takes a few minutes of single-threaded ARPACK, which is why
 
     python tests/golden/make_golden_lsi_slice.py
 
-Output ``lsi_slice_20k.npz`` (committed): singular values (k+1, float64), the full left factor U
-(n x k, float32 storage of the float64 result), V on 4096 sampled peaks, checksums of the input so the GPU
-test can prove it regenerated the same matrix.
+Outputs (committed): ``lsi_slice_20k.npz`` holds the singular values (k+1, float64), V on 4096 evenly spaced
+peaks and checksums of the input so the GPU test can prove it regenerated the same matrix;
+``lsi_slice_20k_U.npz`` holds U on 4096 evenly spaced cells.  Factors are stored as float32 of the float64
+result, and sampled so that each file stays under 1 MB.
 """
 import os
 import sys
@@ -42,10 +43,13 @@ def main():
     np.savez_compressed(
         os.path.join(OUT, "lsi_slice_20k.npz"),
         shape=np.array([N_CELLS, N_PEAKS]), density=DENSITY, topics=TOPICS, seed=SEED, k=K,
-        svalues=r["svalues"], U=r["U"][:, :K].astype(np.float32), V_rows=rows,
+        svalues=r["svalues"], V_rows=rows,
         V_sample=r["LSI"][rows, :K].astype(np.float32),
         nnz=C.nnz, counts_sum=float(C.data.astype(np.float64).sum()),
         tfidf_sum=float(X.data.astype(np.float64).sum()), indices_sum=int(C.indices.astype(np.int64).sum()))
+    cells = np.unique(np.linspace(0, N_CELLS - 1, 4096).astype(np.int64))
+    np.savez_compressed(os.path.join(OUT, "lsi_slice_20k_U.npz"), U_rows=cells,
+                        U_sample=r["U"][cells, :K].astype(np.float32))
 
 
 if __name__ == "__main__":

@@ -134,15 +134,17 @@ def _check_slice(z, n, ad, rtol=1e-4):
     k = int(z["k"])
     s_ref = z["svalues"]
     got_s = ad.uns["lsi"]["stdev"].astype(np.float64) * np.sqrt(n - 1)
-    Uref = z["U"].astype(np.float64)
+    zu = load_golden("lsi_slice_20k_U.npz")
+    Uref = zu["U_sample"].astype(np.float64)
+    Ugot = ad.obsm["X_lsi"][zu["U_rows"]]
     V = ad.varm["LSI"]
     rows = z["V_rows"]
-    # U and singular values: the full gap-aware comparison; V: on the fixture's 4096 sampled peaks, sign-aligned
-    # through U (v_i and u_i flip together)
-    got = {"svalues": got_s, "U": ad.obsm["X_lsi"], "LSI": ad.obsm["X_lsi"]}
+    # singular values: all of them; U: the full gap-aware comparison on the fixture's 4096 sampled cells; V: on its
+    # 4096 sampled peaks, sign-aligned through U (v_i and u_i flip together)
+    got = {"svalues": got_s, "U": Ugot, "LSI": Ugot}
     ref = {"svalues": s_ref[:k], "U": Uref, "LSI": Uref}
     out = compare_lsi(got, ref, rtol=rtol, s_next=s_ref[k])
-    sgn = np.sign(np.sum(ad.obsm["X_lsi"].astype(np.float64) * Uref, axis=0))
+    sgn = np.sign(np.sum(Ugot.astype(np.float64) * Uref, axis=0))
     Vs = V[rows].astype(np.float64) * sgn
     Vr = z["V_sample"].astype(np.float64)
     ext = np.concatenate([s_ref[:k], [s_ref[k]]])

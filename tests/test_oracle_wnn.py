@@ -7,7 +7,6 @@ import scipy.sparse as sp
 
 from conftest import golden_csr, load_golden
 from oracle import _third_party as tp
-from oracle._refload import reference_available
 
 
 def test_exact_search_and_helpers():
@@ -47,23 +46,6 @@ def test_wnn_golden_is_consistent():
     assert Dm.data.min() >= 0 and Dm.data.max() <= np.sqrt(0.5) + 1e-12  # sqrt(0.5 (1 - affinity)), affinity in [0,1]
     Cm = golden_csr(z, "wnn_conn")
     assert (Cm != Cm.T).nnz == 0
-
-
-@pytest.mark.skipif(not reference_available(), reason="needs /root/reference")
-def test_reference_neighbors_reproduces_golden():
-    import sys, os
-    sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
-    from make_golden import wnn_inputs
-    from oracle._refload import load_reference_neighbors
-    md = wnn_inputs()
-    load_reference_neighbors()(md, n_multineighbors=40)
-    z = load_golden("wnn_small.npz")
-    np.testing.assert_allclose(md.obs["rna:mod_weight"].to_numpy(), z["w_rna"], rtol=1e-10)
-    got = sp.csr_matrix(md.obsp["distances"])
-    got.sort_indices()
-    ref = golden_csr(z, "wnn_dist")
-    np.testing.assert_array_equal(got.indices, ref.indices)
-    np.testing.assert_allclose(got.data, ref.data, rtol=1e-10, atol=1e-12)
 
 
 def test_numpy_restatement_reproduces_reference_driver_golden():
